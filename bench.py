@@ -30,6 +30,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (no __pycache__ of the modules it imports)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 TF, TU, TS, TNULL = 196608, 2048, 2552, 2656
@@ -321,6 +322,34 @@ def prefer_host_memory_near_gpu(index):
     return info
 
 
+DUMP_STREAMS = 1024      # streams of the batch (a fixed, seeded sample) whose outputs --dump-outputs writes
+
+
+def dump_outputs(out_dir, a, pkg, device, S, buf, n_calls, buf_start_for):
+    """--dump-outputs: the outputs of the last timed step, one float64 .npy per array.  dabb_process_async hands nothing back to its
+    caller, so a second context with the timed one's configuration repeats the same n_calls steps on the same input and takes the last
+    one through dabb_process (= dabb_process_async + the copies of the step's outputs to the host).  Written for a seeded sample of
+    DUMP_STREAMS streams (streams.npy): every field of the per-stream results, the FIBs, and the sub-channel's logical frames (msc) and
+    superframe (sf)."""
+    c = pkg.Context(n_streams=S, device=device, fft_mode=a.fft_mode, disable_coarse=True, n_subch_slots=1, max_subch_cu=SUBCH_CU,
+                    ofdm_tail_split=-1 if a.no_tail_split else 0)
+    c.select_subchannel(0, SUBCH_CU, BITRATE, eep_profile_a=True, eep_level=3, dabplus=True)
+    for call in range(n_calls - 1):
+        c.process_async(buf.data_ptr(), BUF_LEN, buf_start_for(call), BUF_LEN)
+    out = c.process(buf, BUF_LEN, buf_start_for(n_calls - 1), BUF_LEN, msc_stride=3 * BITRATE, sf_stride=15 * BITRATE)
+    c.close()
+    pick = np.sort(np.random.default_rng(0xD0D0).choice(S, min(S, DUMP_STREAMS), replace=False))
+    r = out["results"][pick]
+    arrays = {"streams": pick, "fibs": out["fibs"][pick], "msc": out["msc"][pick, 0], "sf": out["sf"][pick, 0]}
+    arrays.update({"results_" + f: r[f] for f in r.dtype.names if f != "reserved"})
+    arrays = {k: np.ascontiguousarray(v, np.float64) for k, v in arrays.items()}
+    assert sum(v.nbytes for v in arrays.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    return sorted(arrays)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -338,6 +367,8 @@ def main():
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-tail-split", action="store_true", help="A/B: do not cut the last frames of the OFDM launch into short CTAs")
     ap.add_argument("--cfo-hz", type=float, default=50.0, help="carrier offset of the secondary 'oscillator active' measurement (0 = skip); must keep the 5-frame ring periodic (multiples of 1/0.48 s)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0, a seeded sample of the streams) as DIR/<name>.npy, float64")
     a = ap.parse_args()
     if a.impl == "reference":
         reference_arm(a)
@@ -448,6 +479,9 @@ def main():
     ok_frames = int((r["status"] == 0).sum()); fib_ok = int(sum(bin(int(m)).count("1") for m in r["fib_crc_mask"]))
     lf = int(r["n_logical"][:, 0].sum()); rs_unc = int((r["rs_uncorr_mask"][:, 0] != 0).sum()); rs_ev = int(r["n_rs_events"][:, 0].sum())
     check = {"frames_decoded": ok_frames, "streams": S, "fib_crc_ok": fib_ok, "fibs": 12 * S, "logical_frames": lf, "rs_attempts": rs_ev, "rs_uncorrectable_streams": rs_unc}
+    if a.dump_outputs and rank == 0:
+        names = dump_outputs(a.dump_outputs, a, pkg, local, S, buf, a.warmup + a.steps, buf_start_for)
+        log(f"outputs of the last timed step written to {a.dump_outputs}: {', '.join(names)}")
 
     # ---- per-kernel device times over K more steady-state steps (CUDA events on the library's stream after every launch)
     ctx.profile(True)

@@ -289,6 +289,11 @@ class Ref:
         cw = np.array(cw, np.uint8).copy(); pos = np.zeros(10, np.int32)
         r = self.lib.ref_rs_decode_codeword(_p(cw), _p(pos)); return r, cw, pos
 
+    def rs_decode_codewords(self, cws):
+        """rs_decode_codeword over the rows of cws [n, 120] -> (results [n], corrected codewords [n, 120], positions [n, 10])"""
+        res = [self.rs_decode_codeword(cw) for cw in np.asarray(cws, np.uint8)]
+        return np.array([r[0] for r in res], np.int32), np.stack([r[1] for r in res]), np.stack([r[2] for r in res])
+
     def rs_decode_superframe(self, sf):
         sf = np.array(sf, np.uint8).copy(); c = C.c_int(); u = C.c_int()
         self.lib.ref_rs_decode_superframe(_p(sf), len(sf), C.byref(c), C.byref(u)); return sf, c.value, u.value
@@ -307,6 +312,14 @@ class Ref:
         fec = np.zeros(2 * (n + 1), np.int32); au_err = C.c_int(); good = C.c_int()
         k = self.lib.ref_superframe_filter(_p(frames), n, flen, _p(fec), n + 1, C.byref(au_err), C.byref(good))
         return fec[:2 * k].reshape(-1, 2), au_err.value, good.value
+
+    def fib_dump(self, fibs):
+        """FIBProcessor fed the 32-byte FIBs in order -> its text dump of the database and of the FIG-derived callbacks"""
+        fibs = np.ascontiguousarray(fibs, np.uint8)
+        buf = C.create_string_buffer(1 << 18)
+        n = self.lib.ref_fib_dump(_p(fibs), len(fibs), buf, len(buf))
+        assert n >= 0
+        return buf.value.decode("latin1")
 
     def tii_run(self, nulls, prss):
         """the unmodified TIIDecoder fed frame by frame: nulls [n, 2656], prss [n, 2048] complex64 -> [(comb, pattern, delay_samples, error), ...]"""

@@ -14,6 +14,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <time.h>
 
 typedef struct {
     float* iq; long n;
@@ -111,6 +112,10 @@ int dabb_remove_subchannel(dabb_ctx* c, int32_t first, int32_t count, int32_t sl
 int dabb_process(dabb_ctx* c, const dabb_io* io)
 {
     if (!c || !io || !io->results) return DABB_E_ARG;
+    /* a step of the real library takes time; at least 2 ms here too, so that what the glue does from other threads (the controller's
+     * service selection) lands while its worker is decoding, however fast the host is */
+    const struct timespec step = {0, 2000000};
+    nanosleep(&step, NULL);
     for (int s = 0; s < c->S; s++) {
         mock_stream* z = &c->st[s];
         dabb_frame_result* r = &io->results[s];
